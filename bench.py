@@ -8,6 +8,8 @@ NTT's achieved HBM roofline fraction.
   python bench.py --gpus N --steps K --warmup W            our arm (one process per GPU under torchrun for N > 1)
   python bench.py --impl reference --gpus N --steps K ...  the CPU arm: the oracle ("port" of the reference's
                                                            pure-Go path; Go is not installed) on all host cores
+  python bench.py ... --dump-outputs DIR                   also writes a seeded sample of the last timed step's output
+                                                           (write_dump) for output-for-output comparison of two builds
 
 A "step" = one pass of MulRelinNew + Rescale over a batch of `--batch` synthetic ciphertext pairs per GPU
 (uniform residues, random evaluation key: SURVEY 8(d)). `value` times the device-resident path (inputs already
@@ -44,7 +46,38 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--workload", default="mulrelin", choices=["mulrelin", "bootstrap"],
                     help="bootstrap: BASELINE config 5 -- replay of the op trace of one CKKS bootstrapping (use --preset BOOT_N16QP1767)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write a fixed sample of the last step's output ciphertexts (rank 0) to DIR as .npy files")
+    args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "mulrelin"):
+        ap.error("--dump-outputs needs --impl ours --workload mulrelin")
+    return args
+
+
+# Output sample of --dump-outputs: DUMP_SAMPLES flat positions drawn with a fixed seed, so that two builds given the same
+# arguments (hence the same seeded inputs) can be compared output for output. Residues reach 2^56, past float64's 53-bit
+# mantissa, so each one is stored exactly as its high and low 32-bit halves. 3 float64 arrays x 2^21 entries = 50 MB.
+DUMP_SAMPLES = 1 << 21
+DUMP_SEED = 20261017
+
+
+def dump_sample_index(numel):
+    """Sorted, distinct flat positions into an output of `numel` residues (all of them when it is small)."""
+    import numpy as np
+    if numel <= DUMP_SAMPLES:
+        return np.arange(numel, dtype=np.int64)
+    return np.unique(np.random.default_rng(DUMP_SEED).integers(0, numel, DUMP_SAMPLES, dtype=np.int64))
+
+
+def write_dump(dirname, out_shape, idx, vals):
+    """Writes the sampled residues `vals` (uint64, at flat positions `idx` of an output of shape `out_shape`)."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    vals = np.asarray(vals, dtype=np.uint64)
+    arrays = {"ct_out_hi32": vals >> np.uint64(32), "ct_out_lo32": vals & np.uint64(0xFFFFFFFF), "ct_out_index": idx,
+              "ct_out_shape": np.asarray(out_shape)}
+    for name, arr in arrays.items():
+        np.save(os.path.join(dirname, name + ".npy"), arr.astype(np.float64))
 
 
 # ----------------------------------------------------------------------------------------------------------
@@ -320,6 +353,10 @@ def gpu_main(args):
     t_dev = e0.elapsed_time(e1) * 1e-3
     t_max = D.max_over_ranks(t_dev, dev)
     value = D.job_throughput(B * args.steps, t_dev, dev)
+    dump = None
+    if args.dump_outputs and rank == 0:
+        idx = dump_sample_index(out.numel())
+        dump = (tuple(out.shape), idx, out.reshape(-1)[torch.from_numpy(idx).to(dev)].cpu().numpy().view(np.uint64))
 
     # ---- roofline of the dominant kernel class (NTT): same K steps with the event profiler on --------------------
     roof = None
@@ -439,6 +476,8 @@ def gpu_main(args):
             "config": _config(args, s, world),
             "clocks": clocks, "gpu_launches": int(launches), "e2e": e2e, "roofline": roof, "cpu_baseline": cpu,
         }
+        if dump is not None:
+            write_dump(args.dump_outputs, *dump)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

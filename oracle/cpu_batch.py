@@ -9,7 +9,9 @@ import ctypes
 import hashlib
 import os
 import platform
+import shutil
 import subprocess
+import tempfile
 from typing import Optional, Sequence
 
 import numpy as np
@@ -33,14 +35,25 @@ def _cpu_tag() -> str:
     return hashlib.sha1(flags.encode()).hexdigest()[:10]
 
 
-def build(force: bool = False) -> str:
-    """gcc -O3 -march=native of lattigo_cpu_batch.c (+ the #included lattigo_oracle.c) into oracle/_build/."""
-    out = os.path.join(_HERE, "_build", "liblattigo_cpubatch_%s.so" % _cpu_tag())
-    srcs = [os.path.join(_HERE, "lattigo_cpu_batch.c"), os.path.join(_HERE, "lattigo_oracle.c")]
-    if force or not os.path.exists(out) or any(os.path.getmtime(s) > os.path.getmtime(out) for s in srcs):
+_SRCS = [os.path.join(_HERE, "lattigo_cpu_batch.c"), os.path.join(_HERE, "lattigo_oracle.c")]
+_BUILD = os.path.join(_HERE, "_build")
+
+
+def _target(out_dir: str) -> str:
+    return os.path.join(out_dir, "liblattigo_cpubatch_%s.so" % _cpu_tag())
+
+
+def _stale(out: str) -> bool:
+    return not os.path.exists(out) or any(os.path.getmtime(s) > os.path.getmtime(out) for s in _SRCS)
+
+
+def build(force: bool = False, out_dir: Optional[str] = None) -> str:
+    """gcc -O3 -march=native of lattigo_cpu_batch.c (+ the #included lattigo_oracle.c) into `out_dir` (default oracle/_build/)."""
+    out = _target(out_dir or _BUILD)
+    if force or _stale(out):
         os.makedirs(os.path.dirname(out), exist_ok=True)
         cmd = ["gcc", "-O3", "-march=native", "-fPIC", "-shared", "-pthread", "-ffp-contract=off", "-fno-fast-math",
-               "-Wall", "-Wextra", "-Wno-unused-function", "-o", out, srcs[0]]
+               "-Wall", "-Wextra", "-Wno-unused-function", "-o", out, _SRCS[0]]
         subprocess.check_call(cmd)
     return out
 
@@ -63,7 +76,13 @@ _lib = None
 def lib():
     global _lib
     if _lib is None:
-        L = ctypes.CDLL(build())
+        tmp = None
+        if _stale(_target(_BUILD)):
+            # build() ran on another host CPU, or not at all: compile for this host outside the source tree
+            tmp = tempfile.mkdtemp(prefix="lattigo_cpubatch_")
+        L = ctypes.CDLL(build(out_dir=tmp))
+        if tmp:
+            shutil.rmtree(tmp)
         p, i, u, z = ctypes.c_void_p, ctypes.c_int, ctypes.c_uint64, ctypes.c_size_t
         L.lo_ckks_mulrelin_rescale_batch.argtypes = [ctypes.POINTER(_Plan), p, p, z, p, p, i, i, p, p]
         L.lo_ckks_mulrelin_rescale_batch.restype = ctypes.c_double

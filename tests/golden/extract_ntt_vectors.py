@@ -1,22 +1,23 @@
 """Extracts the golden NTT vectors of the reference's own test-suite
-(/root/reference/ring/ntt_test.go:10-89: six vectors, N in {16..512}, two
-61-bit... actually 59-bit limbs each) into tests/golden/ntt_vectors.json.
+(ring/ntt_test.go:10-89 of tuneinsight/lattigo v6.2.0: six vectors, N in {16..512}, two
+59-bit limbs each) into tests/golden/ntt_vectors.json.
 
-Run once in the build container (the reference tree is not present on the GPU
-box):  python tests/golden/extract_ntt_vectors.py
-Only numeric literals are extracted -- no reference code is copied.
+    python tests/golden/extract_ntt_vectors.py <lattigo checkout>/ring/ntt_test.go
+
+The tests read only the JSON file. Only numeric literals are extracted -- no reference code is copied.
 """
 import json
 import os
 import re
 import sys
 
-REF = sys.argv[1] if len(sys.argv) > 1 else "/root/reference/ring/ntt_test.go"
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "ntt_vectors.json")
 
 
 def main():
-    src = open(REF).read()
+    if len(sys.argv) != 2:
+        sys.exit("usage: python tests/golden/extract_ntt_vectors.py <lattigo v6.2.0 checkout>/ring/ntt_test.go")
+    src = open(sys.argv[1]).read()
     body = src[src.index("var testVector"):]
     body = body[: body.index("\n}\n") + 3]
     # each vector: N, Qis, poly (2 rows), polyNTT (2 rows)

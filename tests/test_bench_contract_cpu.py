@@ -46,6 +46,38 @@ def test_bootstrap_workload_reference_arm_is_declared_unavailable():
     assert line["impl"] == "reference" and "unavailable" in line
 
 
+def test_dump_outputs_sample_is_fixed_exact_and_bounded(tmp_path):
+    """--dump-outputs at the headline shape (64 x 2 x 43 x 2^16 residues): the sampled positions are the same on every run,
+    distinct and in range, residues up to 2^56 - 1 come back exactly from the float64 files, and the files stay under 64 MB."""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    shape = (64, 2, 43, 1 << 16)
+    n = int(np.prod(shape))
+    idx = bench.dump_sample_index(n)
+    assert np.array_equal(idx, bench.dump_sample_index(n))
+    assert (np.diff(idx) > 0).all() and idx[0] >= 0 and idx[-1] < n
+    assert np.array_equal(bench.dump_sample_index(100), np.arange(100))
+    vals = np.random.default_rng(5).integers(0, 1 << 56, len(idx), dtype=np.uint64)
+    vals[:2] = [0, (1 << 56) - 1]
+    bench.write_dump(str(tmp_path), shape, idx, vals)
+    files = {f.name[:-4]: np.load(f) for f in tmp_path.iterdir()}
+    assert sorted(files) == ["ct_out_hi32", "ct_out_index", "ct_out_lo32", "ct_out_shape"]
+    assert all(a.dtype == np.float64 for a in files.values())
+    assert sum(f.stat().st_size for f in tmp_path.iterdir()) <= 64 << 20
+    got = (files["ct_out_hi32"].astype(np.uint64) << np.uint64(32)) | files["ct_out_lo32"].astype(np.uint64)
+    assert np.array_equal(got, vals) and np.array_equal(files["ct_out_index"].astype(np.int64), idx)
+    assert tuple(files["ct_out_shape"].astype(np.int64)) == shape
+
+
+def test_dump_outputs_is_refused_where_nothing_is_dumped(tmp_path):
+    for extra in (["--impl", "reference"], ["--workload", "bootstrap"]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--dump-outputs", str(tmp_path / "d")] + extra,
+                           capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert r.returncode == 2 and "--dump-outputs" in r.stderr
+        assert not (tmp_path / "d").exists()
+
+
 def test_clock_sampler_keeps_the_samples_of_the_timed_region():
     """ClockSampler.stop(t0, t1): only lines that arrived during the timed region count (the poller runs from before the warm-up);
     throttle reasons outside it are not reported, reasons inside it are; a region shorter than the polling period keeps the nearest lines."""
