@@ -310,7 +310,11 @@ int lgpu_rgsw_external_product(lgpu_ctx* ctx, const uint64_t* ct_in, int level_i
 
 /* ---- encryptor / key-generator inner loops and device samplers (core/rlwe/encryptor.go, keygenerator.go, ring/sampler_*.go) ----
  * Samplers: the reference's distributions on Philox4x32-10 counter streams keyed by (seed, stream_id) -- NOT the reference's
- * blake2b-XOF byte stream (sampling/prng.go), which is inherently sequential. Small polynomials are int64 vectors [batch][N]. */
+ * blake2b-XOF byte stream (sampling/prng.go), which is inherently sequential. Small polynomials are int64 vectors [batch][N].
+ * Each (seed, stream_id, sampler kind, limb) has its own counter space: two samplers, or the Q and P rows of a uniform draw,
+ * never read the same random block, and a uniform row does not depend on the level it is drawn at.
+ * Philox with a 64-bit seed is a statistical generator, not a cryptographic one: it suits tests and benchmarks. Production
+ * key material should come from the caller (a host CSPRNG) through the int64 / residue arguments of the functions below. */
 /* ringqp.UniformSampler.Read (ring/sampler_uniform.go:48-100): rows 0..level uniform in [0, q_i). */
 int lgpu_sample_uniform(lgpu_ctx* ctx, int ring, int level, uint64_t seed, uint64_t stream_id, uint64_t* out, int batch,
                         size_t batch_stride, void* stream);

@@ -9,8 +9,8 @@
 //   ringqp.Ring.ExtendBasisSmallNormAndCenter             ring/ringqp/operations.go:325-351 (folded into small_to_rns)
 // Samplers (ring/sampler_uniform.go, sampler_ternary.go, sampler_gaussian.go): same DISTRIBUTIONS, own random streams -- the
 // reference reads a blake2b XOF sequentially (sampling/prng.go), which has no parallel form; here every coefficient owns a
-// Philox4x32-10 counter (seed, stream, polynomial, coefficient, attempt), so a batch of polynomials is sampled in one launch and
-// the result does not depend on the launch geometry.
+// Philox4x32-10 counter (seed, stream, sampler kind, polynomial, coefficient, attempt), so a batch of polynomials is sampled in
+// one launch and the result does not depend on the launch geometry. tests/sampler_model.py restates these kernels bit for bit.
 #include <cmath>
 #include <cstring>
 #include <vector>
@@ -35,12 +35,19 @@ __device__ __forceinline__ Ph4 philox4x32_10(Ph4 c, unsigned k0, unsigned k1) {
     }
     return c;
 }
-struct SampleKey { unsigned k0, k1, stream; };
+// Counter layout {coefficient or draw index, kind << 30 | polynomial, low half of the stream id, attempt} under the key
+// (seed, high half of the stream id): every (seed, stream id, sampler kind, polynomial) has its own counter space, so no two
+// samplers, rings or batch elements ever read the same block. polynomial < 2^30: batch * kMaxRows + limb for the uniform
+// sampler, the batch index otherwise.
+enum SampleKind : unsigned { kUniform = 0, kTernaryP = 1, kTernaryH = 2, kGaussian = 3 };
+struct SampleKey { unsigned k0, k1, stream, kind; };
 __device__ __forceinline__ Ph4 draw(const SampleKey& k, unsigned poly, unsigned coeff, unsigned attempt) {
-    return philox4x32_10(Ph4{coeff, poly, k.stream, attempt}, k.k0, k.k1);
+    return philox4x32_10(Ph4{coeff, k.kind << 30 | poly, k.stream, attempt}, k.k0, k.k1);
 }
 
-// uniform in [0, q) per row: masked 64-bit words, rejected until below q (ring/sampler_uniform.go:48-100)
+// uniform in [0, q) per row: masked 64-bit words, rejected until below q (ring/sampler_uniform.go:48-100). A row draws from the
+// stream of its global limb (Q limbs, then P limbs), so the Q and P rows of one stream id differ and a row does not depend on
+// the level it is drawn at.
 struct UniformParams {
     const LimbConst* limbs; RowMap rm;
     u64* out; size_t rs, bs;
@@ -52,7 +59,7 @@ __global__ void __launch_bounds__(256) sample_uniform_kernel(UniformParams p) {
     const int r = blockIdx.y, b = blockIdx.z;
     const u64 q = p.limbs[p.rm.limb[r]].q;
     const u64 mask = ~0ull >> __clzll((long long)(q - 1));
-    const unsigned poly = (unsigned)b * kMaxRows + (unsigned)r;
+    const unsigned poly = (unsigned)b * kMaxRows + p.rm.limb[r];
     u64 v = 0;
     for (unsigned a = 0;; a++) {
         const Ph4 d = draw(p.key, poly, (unsigned)i, a);
@@ -154,9 +161,10 @@ __global__ void __launch_bounds__(256) gadget_add_kernel(GadgetAddParams p) {
     *dst = cred(*dst + t, L.q);
 }
 
-static SampleKey make_key(u64 seed, u64 stream) {
+static SampleKey make_key(u64 seed, u64 stream, SampleKind kind) {
     SampleKey k;
     k.k0 = (unsigned)seed; k.k1 = (unsigned)(seed >> 32) ^ (unsigned)(stream >> 32) * 0x85EBCA6Bu; k.stream = (unsigned)stream;
+    k.kind = kind;
     return k;
 }
 
@@ -297,7 +305,7 @@ int lgpu_sample_uniform(lgpu_ctx* ctx, int ring, int level, uint64_t seed, uint6
     REQUIRE(out && batch >= 1 && batch <= 65535, "bad argument");
     UniformParams p;
     if (make_rowmap(ctx->c, ring, level, p.rm)) return -1;
-    p.limbs = ctx->c.d_limbs; p.out = (u64*)out; p.rs = ctx->c.N; p.bs = batch_stride; p.key = make_key(seed, stream_id); p.n = ctx->c.N;
+    p.limbs = ctx->c.d_limbs; p.out = (u64*)out; p.rs = ctx->c.N; p.bs = batch_stride; p.key = make_key(seed, stream_id, kUniform); p.n = ctx->c.N;
     count_launch(1);
     sample_uniform_kernel<<<dim3((ctx->c.N + 255) / 256, p.rm.nrows, batch), 256, 0, (cudaStream_t)stream>>>(p);
     LGPU_CUDA_OK(cudaGetLastError());
@@ -312,10 +320,10 @@ int lgpu_sample_ternary(lgpu_ctx* ctx, double p, int hamming_weight, uint64_t se
     if (hamming_weight > 0) {
         REQUIRE(hamming_weight <= N, "ternary sampler: Hamming weight above N");
         const size_t smem = (size_t)((N + 31) / 32) * sizeof(unsigned);
-        sample_ternary_h_kernel<<<batch, 256, smem, (cudaStream_t)stream>>>((long long*)out, N, hamming_weight, make_key(seed, stream_id));
+        sample_ternary_h_kernel<<<batch, 256, smem, (cudaStream_t)stream>>>((long long*)out, N, hamming_weight, make_key(seed, stream_id, kTernaryH));
     } else {
         REQUIRE(p > 0.0 && p <= 1.0, "ternary sampler: P must be in (0, 1]");
-        sample_ternary_p_kernel<<<dim3((N + 255) / 256, batch), 256, 0, (cudaStream_t)stream>>>((long long*)out, N, p, make_key(seed, stream_id));
+        sample_ternary_p_kernel<<<dim3((N + 255) / 256, batch), 256, 0, (cudaStream_t)stream>>>((long long*)out, N, p, make_key(seed, stream_id, kTernaryP));
     }
     LGPU_CUDA_OK(cudaGetLastError());
     return 0;
@@ -327,7 +335,7 @@ int lgpu_sample_gaussian(lgpu_ctx* ctx, double sigma, double bound, uint64_t see
     REQUIRE(sigma > 0.0 && bound >= 1.0 && bound < 9.0e18, "gaussian sampler: sigma / bound out of range");
     const int N = ctx->c.N;
     count_launch(1);
-    sample_gaussian_kernel<<<dim3((N + 255) / 256, batch), 256, 0, (cudaStream_t)stream>>>((long long*)out, N, sigma, bound, make_key(seed, stream_id));
+    sample_gaussian_kernel<<<dim3((N + 255) / 256, batch), 256, 0, (cudaStream_t)stream>>>((long long*)out, N, sigma, bound, make_key(seed, stream_id, kGaussian));
     LGPU_CUDA_OK(cudaGetLastError());
     return 0;
 }

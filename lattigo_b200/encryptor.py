@@ -29,21 +29,20 @@ class Samplers:
         return out
 
     def UniformQP(self, levelQ: int, levelP: int, batch: int = 1, stream_id=None):
-        """A uniform ringqp.Poly block (batch, levelQ+1 + levelP+1, N)."""
-        import torch
+        """A uniform ringqp.Poly block (batch, levelQ+1 + levelP+1, N). Both rings draw from one stream id: the device keys
+        every row by its limb, so the Q and P rows never share random blocks."""
         sid = self._sid(stream_id)
         rows = levelQ + 1 + levelP + 1
-        out = torch.empty((batch, rows, self.ctx.N), dtype=torch.int64, device="cuda:%d" % self.ctx.device)
+        out = self.ctx.new_poly(rows, batch)
         L = _lib.lib()
-        _lib.check(L.lgpu_sample_uniform(self.ctx.h, RING_Q, levelQ, self.seed, 2 * sid, ctypes.c_void_p(out.data_ptr()), batch, rows * self.ctx.N, _stream()))
+        _lib.check(L.lgpu_sample_uniform(self.ctx.h, RING_Q, levelQ, self.seed, sid, _dptr(out), batch, rows * self.ctx.N, _stream()))
         if levelP >= 0:
-            _lib.check(L.lgpu_sample_uniform(self.ctx.h, RING_P, levelP, self.seed, 2 * sid + 1,
+            _lib.check(L.lgpu_sample_uniform(self.ctx.h, RING_P, levelP, self.seed, sid,
                                              ctypes.c_void_p(out.data_ptr() + 8 * (levelQ + 1) * self.ctx.N), batch, rows * self.ctx.N, _stream()))
         return out
 
     def _small(self, batch):
-        import torch
-        return torch.empty((batch, self.ctx.N), dtype=torch.int64, device="cuda:%d" % self.ctx.device)
+        return self.ctx.new_poly(1, batch).view(batch, self.ctx.N)
 
     def Ternary(self, P: float = 0.0, H: int = 0, batch: int = 1, stream_id=None):
         out = self._small(batch)

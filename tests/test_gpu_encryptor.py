@@ -1,5 +1,5 @@
 """GPU side of SURVEY 8(f) rank 3 (csrc/encrypt.cu): the encryptor / key-generator inner loops bit for bit against
-oracle/encryptor.py on the same sampled polynomials, the device samplers' distributions, and an end-to-end check (device-sampled
+oracle/encryptor.py on the same sampled polynomials, the samplers' stream handling, and an end-to-end check (device-sampled
 secret / error / uniform polynomials -> device evaluation key -> key switch -> oracle-side noise measurement)."""
 import numpy as np
 import pytest
@@ -96,38 +96,22 @@ def test_gen_evaluation_key_matches_the_oracle(pw2, lp):
 
 
 def test_samplers_distributions_and_streams():
-    import torch
+    """Wrapper-level stream handling (the kernels themselves are pinned in tests/test_gpu_samplers.py): an explicit stream id
+    reproduces its draw, another id gives another draw, and a polynomial does not depend on the batch it was drawn in."""
     import lattigo_b200 as lb
     logN = 12
     q, p = O.gen_moduli(logN + 1, [55, 45, 30], [61])
     ctx = lb.Context(logN, q, p)
     try:
-        N = 1 << logN
         S = lb.encryptor.Samplers(ctx, seed=0x1234567890ABCDEF)
         u = ctx.to_host(S.UniformQP(2, 0, batch=4, stream_id=7))
-        for i, m in enumerate(q + p):
-            row = u[:, i].astype(np.float64)
-            assert int(u[:, i].max()) < m
-            assert abs(row.mean() / m - 0.5) < 0.02 and abs(row.std() / m - 0.2887) < 0.02
-        assert len(np.unique(u[:, 0])) > 0.99 * 4 * N                       # rows / batch elements do not share a stream
         assert np.array_equal(u, ctx.to_host(S.UniformQP(2, 0, batch=4, stream_id=7)))      # reproducible
         assert not np.array_equal(u, ctx.to_host(S.UniformQP(2, 0, batch=4, stream_id=8)))
         # the counter-based streams do not depend on the batch they were drawn in
         assert np.array_equal(u[:2], ctx.to_host(S.UniformQP(2, 0, batch=2, stream_id=7)))
-        t = S.Ternary(P=0.5, batch=8).cpu().numpy()
-        assert set(np.unique(t)) == {-1, 0, 1}
-        assert abs((t != 0).mean() - 0.5) < 0.02 and abs((t == 1).mean() - (t == -1).mean()) < 0.02
-        for h in (32, N // 2):
-            th = S.Ternary(H=h, batch=3).cpu().numpy()
-            assert ((th != 0).sum(axis=1) == h).all() and set(np.unique(th)) <= {-1, 0, 1}
-            assert abs((th == 1).sum() - (th == -1).sum()) < 6 * np.sqrt(3 * h)
-        g = S.Gaussian(3.2, 19.2, batch=16).cpu().numpy().astype(np.float64)
-        assert np.abs(g).max() <= 19 and abs(g.mean()) < 0.05
-        assert abs(g.std() - np.sqrt(3.2 ** 2 + 1 / 12)) < 0.05            # rounding adds the variance of a unit uniform
-        small = torch.from_numpy(np.array([[-3, 0, 5] + [0] * (N - 3)], dtype=np.int64)).cuda()
-        rq, rp = lb.encryptor.small_poly_to_rns(ctx, small, 2, 0)
-        assert [int(x) for x in ctx.to_host(rq)[0, :, 0]] == [m - 3 for m in q] and int(ctx.to_host(rp)[0, 0, 0]) == p[0] - 3
-        assert int(ctx.to_host(rq)[0, 1, 2]) == 5
+        g = S.Gaussian(3.2, 19.2, batch=3, stream_id=5).cpu().numpy()
+        assert np.array_equal(g[:1], S.Gaussian(3.2, 19.2, batch=1, stream_id=5).cpu().numpy())
+        assert np.array_equal(S.Ternary(H=32, batch=3, stream_id=6).cpu().numpy()[:2], S.Ternary(H=32, batch=2, stream_id=6).cpu().numpy())
     finally:
         ctx.close()
 
