@@ -775,6 +775,12 @@ static int ckks_mulrelin_rescale_chunk(const Ctx* c, int level, const u64* ctA, 
             acc.p[k] = Span{base + nq * N, N, (nq + np) * N};
         }
         if (gadget_product_lazy(c, level, CSpan{d2, N, nq * N}, rlk, acc, batch, st)) return -1;
+        // LGPU_FZ_RESCALE (default 1): ModDown and Rescale as one pass (one basis extension and one transform per output row, see
+        // moddown_ntt_fused); 0 runs them as two passes through d0
+        static const int fz_rescale = [] { const char* e = getenv("LGPU_FZ_RESCALE"); return e ? atoi(e) : 1; }();
+        if (nb_rescales == 1 && fz_rescale)
+            return moddown_ntt_fused(c, level, rlk.levelP, accb.p, (size_t)batch * (nq + np) * N, (nq + np) * N, d0, (size_t)batch * nq * N, nq * N,
+                                     out, (nq - 1) * N, 2 * (nq - 1) * N, 2, batch, st, 1);
         // d0, d1 are consecutive [comp][batch][nq][N] blocks: out = d + ModDown(acc), in place
         if (moddown_ntt_fused(c, level, rlk.levelP, accb.p, (size_t)batch * (nq + np) * N, (nq + np) * N, d0, (size_t)batch * nq * N, nq * N,
                               d0, (size_t)batch * nq * N, nq * N, 2, batch, st)) return -1;

@@ -77,7 +77,7 @@ int gadget_product_multiple_p_fused(const Ctx* c, int levelQ, CSpan cx, CSpan cx
 
 bool fz_applicable(const Ctx* c, int levelQ, int levelP);
 int moddown_ntt_fused(const Ctx* c, int levelQ, int levelP, const u64* acc, size_t acc_cs, size_t acc_bs, const u64* D, size_t d_cs, size_t d_bs,
-                      u64* out, size_t o_cs, size_t o_bs, int ncomp, int batch, cudaStream_t st);
+                      u64* out, size_t o_cs, size_t o_bs, int ncomp, int batch, cudaStream_t st, int rescale = 0);
 int div_round_last_ntt_fused(const Ctx* c, int level, const u64* X, size_t x_cs, size_t x_bs, u64* out, size_t o_cs, size_t o_bs,
                              int ncomp, int batch, cudaStream_t st);
 

@@ -89,6 +89,10 @@ struct Ctx {
     u64* d_blob = nullptr;
     std::vector<ModUpSet> muc_QtoP;  // [levelQ]: Q[:levelQ+1] -> P (all)
     std::vector<ModUpSet> muc_PtoQ;  // [levelP]: P[:levelP+1] -> Q (all)
+    // [levelP]: muc_PtoQ with every target-side constant (qoverqimodp, vtimesqmodp, half_t, c_plain) multiplied by
+    // P^-1 mod q_j, P = p_0..p_levelP; source-side offsets are those of muc_PtoQ. The extension it evaluates is P^-1 ModUp(x)
+    // (used by the ModDown + Rescale tail, which needs that product and nothing else)
+    std::vector<ModUpSet> muc_PtoQ_pinv;
     // decomposer sets, ring/basis_extension.go:333-373: index (nbPi-2, digit, decompLvl)
     std::vector<std::vector<std::vector<ModUpSet>>> muc_dec;
     // modDownConstants: [levelP][i] (PtoQ) and [levelQ][j] (QtoP), Montgomery form  (:25-49)

@@ -141,15 +141,17 @@ struct KsStridedParams {
     int single_rule;  // see KsPrepParams
     int src_limb0;    // global limb of source row 0 (single-limb rule only)
     int split23;      // 1: full digits whose sources are all FP64-pipe primes take ks_ext_split on the FP64 target rows (LGPU_K2_SPLIT)
-    // PRO_BCAST (rescale): e = cred(bc[x] + bc_add, bc_q) + s0[launch row]
+    // PRO_BCAST (rescale): e = cred(bc[x] + bc_add, bc_q) + s0[launch row]; PRO_MODUP_BCAST adds the same term to the extension
     const u64* bc; size_t bc_bs; u64 bc_add, bc_q;
     u64 s0[kMaxRows];
     KsDigit dg[kMaxDigits];
 };
 
 // ext value of one coefficient for target limb (q, qinv): reference formula of multSum + centring, reduced to < 3q.
-template <int NSMAX>
-__device__ __forceinline__ u64 ks_ext(const u64 (&y)[NSMAX], int nS, int v, const u64* c, const u64* vt, u64 half_t, u64 q, u64 qinv) {
+// BC: plus a broadcast term bc < 2q, canonical (r + q - half_t < 4q, so the sum is below 6q < 8q, q < 2^61).
+template <int NSMAX, bool BC = false>
+__device__ __forceinline__ u64 ks_ext(const u64 (&y)[NSMAX], int nS, int v, const u64* c, const u64* vt, u64 half_t, u64 q, u64 qinv,
+                                      u64 bc = 0) {
     // 128-bit accumulation through one __int128 so that the partial products chain on IMAD.WIDE / IADD3.X carries
     unsigned __int128 acc = 0;
 #pragma unroll
@@ -158,7 +160,15 @@ __device__ __forceinline__ u64 ks_ext(const u64 (&y)[NSMAX], int nS, int v, cons
     const u64 rlo = (u64)acc, rhi = (u64)(acc >> 64);
     const u64 hhi = mulhi64(rlo * qinv, q);
     u64 r = rhi - hhi + q + vt[v];
+    if (BC) return csub_lt8q(r + q - half_t + bc, q);
     return cred(r + q - half_t, q);
+}
+
+// The Rescale broadcast term of PRO_BCAST, (c_L + floor(q_L/2) mod q_L) + (q - floor(q_L/2) mod q) < q_L + q, brought below 2q for the
+// merged prologue: reduced when the last modulus is above the target prime, where q_L + q could exceed the 8q the integer butterflies accept
+__device__ __forceinline__ u64 bcast_lt2q(u64 c, u64 bc_add, u64 bc_q, u64 s0, u64 q, u64 bred_hi) {
+    const u64 e = cred(c + bc_add, bc_q) + s0;
+    return bc_q > q ? bred_add(e, q, bred_hi) : e;
 }
 
 // The same residue when every source prime of the digit AND the target prime are FP64-pipe primes (below 2^46.3), as a lazy double in
@@ -174,9 +184,11 @@ __device__ __forceinline__ u64 mad_wide(u32 a, u32 b, u64 c) {
     asm("mad.wide.u32 %0, %1, %2, %3;" : "=l"(r) : "r"(a), "r"(b), "l"(c));
     return r;
 }
-template <int NSMAX>
+// BC: plus a broadcast term 0 <= bc < 2q < 2^48 before the last reduction; the sum stays an exact integer below 2^52 (A < 2^51,
+// |vt - half_t| < q, |t| < 0.66q, see above), so the result keeps the (-0.66q, 0.66q) range.
+template <int NSMAX, bool BC = false>
 __device__ __forceinline__ double ks_ext_split(const u64 (&y)[NSMAX], const u32 (&c0)[NSMAX], const u32 (&c1)[NSMAX], const u32 (&d0)[NSMAX],
-                                               const u32 (&d1)[NSMAX], double vtb, double fq, double fqinv) {
+                                               const u32 (&d1)[NSMAX], double vtb, double fq, double fqinv, double bc = 0.0) {
     u64 A = 0, B = 0;
 #pragma unroll
     for (int i = 0; i < NSMAX; i++) {
@@ -189,10 +201,13 @@ __device__ __forceinline__ double ks_ext_split(const u64 (&y)[NSMAX], const u32 
     const double ab = __longlong_as_double((long long)(A | 0x4330000000000000ull));                 // 2^52 + A
     const double bb = __longlong_as_double((long long)(B | 0x4330000000000000ull));                 // 2^52 + B
     const double t = fp_reduce(__fma_rn(bb, 8388608.0, -37778931862957161709568.0), fq, fqinv);     // (2^52 + B) 2^23 - 2^75 = B 2^23, exact
+    if (BC) return fp_reduce(__dadd_rn(__dadd_rn(__dadd_rn(ab, vtb), t), bc), fq, fqinv);
     return fp_reduce(__dadd_rn(__dadd_rn(ab, vtb), t), fq, fqinv);                                  // (2^52 + A) + (vt - half_t - 2^52), exact
 }
 
-enum { PRO_MODUP = 0, PRO_BCAST = 1 };
+// K2 prologues: PRO_MODUP the basis extension, PRO_BCAST the Rescale broadcast of the last row, PRO_MODUP_BCAST their sum (the merged
+// ModDown + Rescale tail: P^-1 ModUp with the constants of Ctx::muc_PtoQ_pinv, plus bcast_lt2q; canonical, see ks_ext)
+enum { PRO_MODUP = 0, PRO_BCAST = 1, PRO_MODUP_BCAST = 2 };
 #ifndef KS_STRIDED_MINB
 #define KS_STRIDED_MINB 5
 #endif
@@ -223,10 +238,10 @@ __global__ void __launch_bounds__(256, KS_STRIDED_MINB) ks_strided_kernel(KsStri
     const KsDigit dg = p.dg[d];
     const int r0 = d * p.k;
     const int nS = dg.nS;
-    if (PRO == PRO_MODUP && p.skip_own && row < p.nq && row >= r0 && row < r0 + nS) return;   // own rows come from the NTT input
+    if (PRO != PRO_BCAST && p.skip_own && row < p.nq && row >= r0 && row < r0 + nS) return;   // own rows come from the NTT input
     const LimbConst L = p.limbs[limb];
     const bool fpsum = FP && PRO == PRO_MODUP && dg.fp_src == 2 && (nS > 1 || !p.single_rule);
-    if (PRO == PRO_MODUP) {
+    if (PRO != PRO_BCAST) {
         if (threadIdx.x < nS) s_c[threadIdx.x] = p.blob[(fpsum ? dg.off_cp : dg.off_c) + (size_t)limb * dg.ldc + threadIdx.x];
         if (threadIdx.x <= nS) s_vt[threadIdx.x] = p.blob[dg.off_vt + (size_t)limb * (dg.ldc + 1) + threadIdx.x];
     }
@@ -293,10 +308,13 @@ __global__ void __launch_bounds__(256, KS_STRIDED_MINB) ks_strided_kernel(KsStri
             for (int k = 0; k < R; k++) e[k] = bred_add(e[k], q, L.bred_hi);
         }
     } else {
+    constexpr bool BC = PRO == PRO_MODUP_BCAST;
     const bool multi = nS > 1 || !p.single_rule;
     const u64 half_t = multi ? p.blob[dg.off_half_t + limb] : 0;
     const u64* Y = p.Y + (size_t)b * p.y_bs + (size_t)r0 * N;
     const unsigned char* V = p.V + (size_t)b * p.v_bs + (size_t)d * N;
+    const u64* bc = BC ? p.bc + (size_t)b * p.bc_bs : nullptr;
+    const u64 s0 = BC ? p.s0[blockIdx.y] : 0;
     if (multi) {
 #pragma unroll
         for (int k = 0; k < R; k++) {
@@ -304,7 +322,8 @@ __global__ void __launch_bounds__(256, KS_STRIDED_MINB) ks_strided_kernel(KsStri
             u64 y[NSMAX];
 #pragma unroll
             for (int i = 0; i < NSMAX; i++) y[i] = i < nS ? Y[(size_t)i * N + x] : 0;
-            e[k] = ks_ext<NSMAX>(y, nS, (int)V[x], s_c, s_vt, half_t, q, qinv);
+            const u64 t = BC ? bcast_lt2q(bc[x], p.bc_add, p.bc_q, s0, q, L.bred_hi) : 0;
+            e[k] = ks_ext<NSMAX, BC>(y, nS, (int)V[x], s_c, s_vt, half_t, q, qinv, t);
         }
     } else {
         // single-limb digit (ring/basis_extension.go:402-436): centre around q_src/2, reduce, restore the sign
@@ -316,6 +335,7 @@ __global__ void __launch_bounds__(256, KS_STRIDED_MINB) ks_strided_kernel(KsStri
             if (neg) c = qs - c;
             const u64 t = bred_add(c, q, L.bred_hi);
             e[k] = neg ? q - t : t;
+            if (BC) e[k] += bcast_lt2q(bc[k * stride + l], p.bc_add, p.bc_q, s0, q, L.bred_hi);     // < 3q
         }
     }
     }
@@ -361,13 +381,17 @@ __global__ void __launch_bounds__(256, KS_STRIDED_MINB) ks_strided_kernel(KsStri
 // Here a CTA owns 64 strided columns (l) x all R strided coefficients and stages that y/v tile in shared memory once
 // for J = 4 target rows (thread = (column, target row)): L2 traffic drops 4x, the y reads become conflict-free /
 // broadcast shared-memory loads. Multi-source digits only (the single-limb rule keeps the plain kernel).
+// BC: prologue PRO_MODUP_BCAST (one digit: the ModDown extension, plus the Rescale broadcast term of the column).
 // ------------------------------------------------------------------------------------------------------------
-template <int RL, int NSMAX, bool FP, bool CORR = true>
+template <int RL, int NSMAX, bool FP, bool CORR = true, bool BC = false>
 __global__ void __launch_bounds__(256, KS_STRIDED_J4_MINB) ks_strided_j4_kernel(KsStridedParams p) {
     constexpr int R = 1 << RL, J = KS_J, LB = 256 / J;
     extern __shared__ u64 dsm[];
     u64* s_y = dsm;                                                        // [NSMAX][R][LB]
     unsigned char* s_v = reinterpret_cast<unsigned char*>(dsm + NSMAX * R * LB);   // [R][LB]
+    // BC: this thread's broadcast terms [R][256], formed before the extension so that their operands are not live across it (with them
+    // live the R = 16 instantiations spill several times more than without)
+    u64* s_bt = dsm + NSMAX * R * LB + R * LB / 8;
     __shared__ u64 s_c[J][NSMAX];
     __shared__ u64 s_vt[J][NSMAX + 1];
     __shared__ u64 s_c2[FP ? J : 1][NSMAX];              // split path: c 2^23 mod q
@@ -413,6 +437,12 @@ __global__ void __launch_bounds__(256, KS_STRIDED_J4_MINB) ks_strided_j4_kernel(
             if (lx < nS) s_c[jj][lx] = p.blob[dg.off_c + (size_t)limb * dg.ldc + lx];
             if (lx <= nS) s_vt[jj][lx] = p.blob[dg.off_vt + (size_t)limb * (dg.ldc + 1) + lx];
         }
+        if (BC) {
+            const u64* bc = p.bc + (size_t)b * p.bc_bs + l0 + lx;
+            const u64 q = p.limbs[limb].q, bh = p.limbs[limb].bred_hi, s0 = p.s0[jrow];
+#pragma unroll
+            for (int k = 0; k < R; k++) s_bt[k * 256 + tid] = bcast_lt2q(bc[k * stride], p.bc_add, p.bc_q, s0, q, bh);
+        }
     }
     __syncthreads();
     if (!valid) return;
@@ -440,7 +470,8 @@ __global__ void __launch_bounds__(256, KS_STRIDED_J4_MINB) ks_strided_j4_kernel(
                 u64 y[NSMAX];
 #pragma unroll
                 for (int i = 0; i < NSMAX; i++) y[i] = s_y[(i * R + k) * LB + lx];
-                x[k] = ks_ext_split<NSMAX>(y, c0, c1, d0, d1, s_vtd[jj][s_v[k * LB + lx]], fq, fqinv);
+                const double t = BC ? u2d(s_bt[k * 256 + tid]) : 0.0;
+                x[k] = ks_ext_split<NSMAX, BC>(y, c0, c1, d0, d1, s_vtd[jj][s_v[k * LB + lx]], fq, fqinv, t);
             }
 #pragma unroll
             for (int u = 0; u < RL; u++) {
@@ -462,7 +493,8 @@ __global__ void __launch_bounds__(256, KS_STRIDED_J4_MINB) ks_strided_j4_kernel(
             u64 y[NSMAX];
 #pragma unroll
             for (int i = 0; i < NSMAX; i++) y[i] = s_y[(i * R + k) * LB + lx];
-            e[k] = ks_ext<NSMAX>(y, NSMAX, (int)s_v[k * LB + lx], s_c[jj], s_vt[jj], half_t, q, qinv);
+            const u64 t = BC ? s_bt[k * 256 + tid] : 0;
+            e[k] = ks_ext<NSMAX, BC>(y, NSMAX, (int)s_v[k * LB + lx], s_c[jj], s_vt[jj], half_t, q, qinv, t);
         }
     } else {
 #pragma unroll
@@ -470,7 +502,8 @@ __global__ void __launch_bounds__(256, KS_STRIDED_J4_MINB) ks_strided_j4_kernel(
             u64 y[NSMAX];
 #pragma unroll
             for (int i = 0; i < NSMAX; i++) y[i] = i < nS ? s_y[(i * R + k) * LB + lx] : 0;
-            e[k] = ks_ext<NSMAX>(y, nS, (int)s_v[k * LB + lx], s_c[jj], s_vt[jj], half_t, q, qinv);
+            const u64 t = BC ? s_bt[k * 256 + tid] : 0;
+            e[k] = ks_ext<NSMAX, BC>(y, nS, (int)s_v[k * LB + lx], s_c[jj], s_vt[jj], half_t, q, qinv, t);
         }
     }
     if constexpr (FP) {
@@ -1036,13 +1069,13 @@ bool ks_fused_applicable(const Ctx* c, int levelQ, const GadgetCt& evk) {
     return true;
 }
 
-template <int RL, int NSMAX, bool FP, bool CORR>
+template <int RL, int NSMAX, bool FP, bool CORR, bool BC>
 static int ks_launch_j4(const KsStridedParams& p, dim3 grid, cudaStream_t st) {
     constexpr int R = 1 << RL;
     constexpr int LB = 256 / KS_J;
-    const size_t smem = (size_t)NSMAX * R * LB * sizeof(u64) + (size_t)R * LB;
-    LGPU_CUDA_OK(cudaFuncSetAttribute(ks_strided_j4_kernel<RL, NSMAX, FP, CORR>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    ks_strided_j4_kernel<RL, NSMAX, FP, CORR><<<dim3(grid.x * KS_J, (grid.y + KS_J - 1) / KS_J, grid.z), 256, smem, st>>>(p);
+    const size_t smem = (size_t)NSMAX * R * LB * sizeof(u64) + (size_t)R * LB + (BC ? (size_t)R * 256 * sizeof(u64) : 0);
+    LGPU_CUDA_OK(cudaFuncSetAttribute(ks_strided_j4_kernel<RL, NSMAX, FP, CORR, BC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    ks_strided_j4_kernel<RL, NSMAX, FP, CORR, BC><<<dim3(grid.x * KS_J, (grid.y + KS_J - 1) / KS_J, grid.z), 256, smem, st>>>(p);
     LGPU_CUDA_OK(cudaGetLastError());
     return 0;
 }
@@ -1050,12 +1083,13 @@ static int ks_launch_j4(const KsStridedParams& p, dim3 grid, cudaStream_t st) {
 // CORR: the integer rows of the launch need the lazy-correction schedule (some prime above 2^57); ignored for FP64 rows
 template <bool FP, int PRO = PRO_MODUP, bool CORR = true>
 static int ks_launch_strided(int rl, int nsmax, const KsStridedParams& p, dim3 grid, cudaStream_t st) {
-    if constexpr (PRO == PRO_MODUP) {
+    if constexpr (PRO != PRO_BCAST) {
+        constexpr bool BC = PRO == PRO_MODUP_BCAST;
         static const int j4 = [] { const char* e = getenv("LGPU_K2_J4"); return e ? atoi(e) : 1; }();
         bool multi = j4 != 0 && rl <= 4;                       // R = 32 (N = 2^17) would need 2 x 66 KB of shared memory
         for (int d = 0; d < p.nd; d++) multi = multi && (p.dg[d].nS > 1 || !p.single_rule);
         if (multi) {
-#define KS_J4(RLV) case RLV: return nsmax <= 4 ? ks_launch_j4<RLV, 4, FP, CORR>(p, grid, st) : ks_launch_j4<RLV, 8, FP, CORR>(p, grid, st);
+#define KS_J4(RLV) case RLV: return nsmax <= 4 ? ks_launch_j4<RLV, 4, FP, CORR, BC>(p, grid, st) : ks_launch_j4<RLV, 8, FP, CORR, BC>(p, grid, st);
             switch (rl) { KS_J4(1) KS_J4(2) KS_J4(3) KS_J4(4) default: break; }
 #undef KS_J4
         }
@@ -1229,6 +1263,9 @@ int gadget_product_multiple_p_fused(const Ctx* c, int levelQ, CSpan cx, CSpan cx
 // chunk pass with an element-wise epilogue: out = CRed( MRed(x + 2q - a, s) [+ d] ), x = NTT(P1 row).
 // Used by the fused ModDown (a = accumulator Q rows, s = -P^-1, d = the other summand of the ciphertext) and the
 // fused rescale (a = input rows, s = RescaleConstants): SubThenMulScalarMontgomeryTwoModulus, ring/vec_ops.go:752.
+// RS (merged ModDown + Rescale tail): out = CRed( MRed(x + 2q - d, s) + MRed(a, s2) ) = ((d - x) q_L^-1 + a P^-1 q_L^-1) mod q with
+// s = RescaleConstants, s2 = MForm(P^-1 q_L^-1), x = NTT(P^-1 ModUp + broadcast term), a the accumulator, d the other summand (or 0).
+// Both MReds are canonical (a < q, s < q), so the sum is below 2q.
 // Buffers with a (component, batch) structure are addressed as  z -> (z / nb) * cs + (z % nb) * bs.
 // ------------------------------------------------------------------------------------------------------------
 struct FzChunkParams {
@@ -1241,9 +1278,17 @@ struct FzChunkParams {
     int nb, logN;
     int wide;                 // 1: A / D / out are 32-byte aligned -> 256-bit accesses in fz_chunk_epi_fp8_kernel (LGPU_K3_WIDE)
     u64 s[kMaxRows];
+    u64 s2[kMaxRows];         // RS only
 };
 
-template <bool FP>
+template <bool RS>
+__device__ __forceinline__ u64 fz_epi(u64 x, u64 a, u64 d, bool has_d, u64 sc, u64 sc2, u64 q, u64 qinv) {
+    if (RS) return cred(mred(x + (q << 1) - d, sc, q, qinv) + mred(a, sc2, q, qinv), q);
+    const u64 r = mred(x + (q << 1) - a, sc, q, qinv);
+    return has_d ? cred(r + d, q) : r;
+}
+
+template <bool FP, bool RS>
 __global__ void __launch_bounds__(256, 2) fz_chunk_epi_kernel(FzChunkParams p) {
     constexpr int CL = 12, T = 256;
     extern __shared__ u64 smem[];
@@ -1254,8 +1299,8 @@ __global__ void __launch_bounds__(256, 2) fz_chunk_epi_kernel(FzChunkParams p) {
     const LimbConst L = p.limbs[limb];
     const int s1 = p.logN - CL;
     const int N = 1 << p.logN;
-    const u64 q = L.q, qinv = L.qinv, twoq = q << 1;
-    const u64 sc = p.s[blockIdx.y];
+    const u64 q = L.q, qinv = L.qinv;
+    const u64 sc = p.s[blockIdx.y], sc2 = RS ? p.s2[blockIdx.y] : 0;
     const int zc = z / p.nb, zb = z % p.nb;
     const size_t roff = (size_t)row * N + ((size_t)chunk << CL);
     const u64* src = p.P1 + (size_t)z * p.p1_bs + roff;
@@ -1303,15 +1348,14 @@ __global__ void __launch_bounds__(256, 2) fz_chunk_epi_kernel(FzChunkParams p) {
                 x = sm[pad_idx(idx)];
                 x = x >= L.kq ? x - L.kq : x;
             }
-            u64 r = mred(x + twoq - a[j], sc, q, qinv);
-            if (D) r = cred(r + d[j], q);
-            out[idx] = r;
+            out[idx] = fz_epi<RS>(x, a[j], d[j], D != nullptr, sc, sc2, q, qinv);
         }
     }
 }
 
 // high-occupancy FP64 variant of the same kernel (512 threads x 8 elements, last round and epilogue in registers,
 // see ks_chunk_mac_fp8r_kernel)
+template <bool RS>
 __global__ void __launch_bounds__(512, 2) fz_chunk_epi_fp8_kernel(FzChunkParams p) {
     constexpr int CL = 12, T = 512;
     extern __shared__ u64 smem[];
@@ -1322,11 +1366,11 @@ __global__ void __launch_bounds__(512, 2) fz_chunk_epi_fp8_kernel(FzChunkParams 
     const LimbConst L = p.limbs[limb];
     const int s1 = p.logN - CL;
     const int N = 1 << p.logN;
-    const u64 q = L.q, qinv = L.qinv, twoq = q << 1;
+    const u64 q = L.q, qinv = L.qinv;
     const double fq = L.fq, fqinv = L.fqinv;
     const double off52 = __dmul_rn((double)(10 + p.logN), fq) + 4503599627370496.0;   // (10 + logN) q + 2^52, exact
     const double* tw = L.ftw_fwd;
-    const u64 sc = p.s[blockIdx.y];
+    const u64 sc = p.s[blockIdx.y], sc2 = RS ? p.s2[blockIdx.y] : 0;
     const int zc = z / p.nb, zb = z % p.nb;
     const size_t roff = (size_t)row * N + ((size_t)chunk << CL);
     const u64* src = p.P1 + (size_t)z * p.p1_bs + roff;
@@ -1381,9 +1425,8 @@ __global__ void __launch_bounds__(512, 2) fz_chunk_epi_fp8_kernel(FzChunkParams 
     for (int j = 0; j < 4; j++) {
         const u64 xa = KS_LAZY_X ? fp_biased_u64(x[2 * j], off52) : fp_canon(x[2 * j], fq, fqinv);
         const u64 xb = KS_LAZY_X ? fp_biased_u64(x[2 * j + 1], off52) : fp_canon(x[2 * j + 1], fq, fqinv);
-        r[j].x = mred(xa + twoq - a[j].x, sc, q, qinv);
-        r[j].y = mred(xb + twoq - a[j].y, sc, q, qinv);
-        if (D) { r[j].x = cred(r[j].x + d[j].x, q); r[j].y = cred(r[j].y + d[j].y, q); }
+        r[j].x = fz_epi<RS>(xa, a[j].x, d[j].x, D != nullptr, sc, sc2, q, qinv);
+        r[j].y = fz_epi<RS>(xb, a[j].y, d[j].y, D != nullptr, sc, sc2, q, qinv);
     }
     if (p.wide) {
         st256(out + 8 * tid, r[0].x, r[0].y, r[1].x, r[1].y);
@@ -1395,7 +1438,7 @@ __global__ void __launch_bounds__(512, 2) fz_chunk_epi_fp8_kernel(FzChunkParams 
 }
 
 // integer-row variant of fz_chunk_epi_fp8_kernel (512 threads x 8 elements, last round and epilogue in registers)
-template <bool CORR>
+template <bool CORR, bool RS>
 __global__ void __launch_bounds__(512, 2) fz_chunk_epi_int8_kernel(FzChunkParams p) {
     constexpr int CL = 12, T = 512;
     extern __shared__ u64 smem[];
@@ -1409,7 +1452,7 @@ __global__ void __launch_bounds__(512, 2) fz_chunk_epi_int8_kernel(FzChunkParams
     const u64 q = L.q, qinv = L.qinv, twoq = q << 1, nq = 0ull - q, kq = L.kq;
     const unsigned mask = L.fwd_mask;
     const ulonglong2* tw = L.tw_fwd;
-    const u64 sc = p.s[blockIdx.y];
+    const u64 sc = p.s[blockIdx.y], sc2 = RS ? p.s2[blockIdx.y] : 0;
     const int zc = z / p.nb, zb = z % p.nb;
     const size_t roff = (size_t)row * N + ((size_t)chunk << CL);
     const u64* src = p.P1 + (size_t)z * p.p1_bs + roff;
@@ -1443,14 +1486,13 @@ __global__ void __launch_bounds__(512, 2) fz_chunk_epi_int8_kernel(FzChunkParams
         u64 xa = x[2 * j], xb = x[2 * j + 1];
         xa = xa >= kq ? xa - kq : xa; xb = xb >= kq ? xb - kq : xb;
         ulonglong2 r;
-        r.x = mred(xa + twoq - a[j].x, sc, q, qinv);
-        r.y = mred(xb + twoq - a[j].y, sc, q, qinv);
-        if (D) { r.x = cred(r.x + d[j].x, q); r.y = cred(r.y + d[j].y, q); }
+        r.x = fz_epi<RS>(xa, a[j].x, d[j].x, D != nullptr, sc, sc2, q, qinv);
+        r.y = fz_epi<RS>(xb, a[j].y, d[j].y, D != nullptr, sc, sc2, q, qinv);
         *reinterpret_cast<ulonglong2*>(out + 8 * tid + 2 * j) = r;
     }
 }
 
-template <bool FP, bool CORR = true>
+template <bool FP, bool CORR = true, bool RS = false>
 static int fz_launch_chunk(const FzChunkParams& p, dim3 grid, cudaStream_t st) {
     const size_t smem = (size_t)(4096 + 256 + 8) * sizeof(u64);
     static const int v8 = [] { const char* e = getenv("LGPU_FZ_VARIANT"); return e ? atoi(e) : 8; }();
@@ -1461,27 +1503,34 @@ static int fz_launch_chunk(const FzChunkParams& p, dim3 grid, cudaStream_t st) {
         FzChunkParams pw = p;
         pw.wide = k3wide && ((reinterpret_cast<uintptr_t>(p.A) | reinterpret_cast<uintptr_t>(p.D) | reinterpret_cast<uintptr_t>(p.out)) & 31u) == 0 &&
                   ((p.a_cs | p.a_bs | p.d_cs | p.d_bs | p.o_cs | p.o_bs) & 3u) == 0;
-        fz_chunk_epi_fp8_kernel<<<grid, 512, smem, st>>>(pw);
+        fz_chunk_epi_fp8_kernel<RS><<<grid, 512, smem, st>>>(pw);
         LGPU_CUDA_OK(cudaGetLastError());
         return 0;
     }
     if (!FP && v8 == 8 && vec_ok) {
-        fz_chunk_epi_int8_kernel<CORR><<<grid, 512, smem, st>>>(p);
+        fz_chunk_epi_int8_kernel<CORR, RS><<<grid, 512, smem, st>>>(p);
         LGPU_CUDA_OK(cudaGetLastError());
         return 0;
     }
-    fz_chunk_epi_kernel<FP><<<grid, 256, smem, st>>>(p);
+    fz_chunk_epi_kernel<FP, RS><<<grid, 256, smem, st>>>(p);
     LGPU_CUDA_OK(cudaGetLastError());
     return 0;
 }
 
-static void split_rows(const Ctx* c, int limb0, int nrows, RowMap& fp, RowMap& in) {
+// Splits `rows` into FP64-pipe rows and integer rows.
+static void split_fp(const Ctx* c, const RowMap& rows, RowMap& fp, RowMap& in) {
     fp.nrows = in.nrows = 0;
-    for (int r = 0; r < nrows; r++) {
-        const int limb = limb0 + r;
-        RowMap& dst = (c->h_limbs[limb].fp_ok && fp64_ntt_supported(c)) ? fp : in;
-        dst.limb[dst.nrows] = (unsigned char)limb; dst.drow[dst.nrows] = (unsigned char)r; dst.nrows++;
+    for (int r = 0; r < rows.nrows; r++) {
+        RowMap& dst = (c->h_limbs[rows.limb[r]].fp_ok && fp64_ntt_supported(c)) ? fp : in;
+        dst.limb[dst.nrows] = rows.limb[r]; dst.drow[dst.nrows] = rows.drow[r]; dst.nrows++;
     }
+}
+
+static RowMap q_rows(int limb0, int nrows) {
+    RowMap rm;
+    rm.nrows = nrows;
+    for (int r = 0; r < nrows; r++) { rm.limb[r] = (unsigned char)(limb0 + r); rm.drow[r] = (unsigned char)r; }
+    return rm;
 }
 
 bool fz_applicable(const Ctx* c, int levelQ, int levelP) {
@@ -1491,25 +1540,71 @@ bool fz_applicable(const Ctx* c, int levelQ, int levelP) {
     return true;
 }
 
+// K2 strided pass with prologue PRO into sp.P1, then the chunk-pass epilogue (cp) over the Q rows `rows`: FP64 rows on `st`, integer rows
+// on the side stream. consts(rm) fills the per-launch-row constants (sp.s0, cp.s, cp.s2) of one row class before its launches;
+// epi_words: algorithmic words per coefficient of the epilogue.
+template <int PRO, bool RS, class F>
+static int fz_tail(const Ctx* c, const RowMap& rows, int nsmax, KsStridedParams& sp, FzChunkParams& cp, int Z, double epi_words, F consts,
+                   cudaStream_t st) {
+    const size_t N = c->N;
+    const int s1 = c->logN - 12;
+    const unsigned gx = (unsigned)(((N >> s1) + 255) / 256);
+    const unsigned chunks = (unsigned)(N >> 12);
+    RowMap fp, in;
+    split_fp(c, rows, fp, in);
+    cudaStream_t sint = fork_side(c, st, fp.nrows > 0 && in.nrows > 0);
+    RowMap in_c, in_n;
+    split_by_corr(c, in, in_c, in_n);
+    for (int pass = 0; pass < 2; pass++) {
+        const RowMap& ir = pass ? in_n : in_c;
+        if (!ir.nrows) continue;
+        consts(ir);
+        { ProfScope ps(LGPU_KCLASS_FUSED, sint, 8.0 * N * Z * ir.nrows, 1);
+          sp.rm = ir;
+          if (pass ? ks_launch_strided<false, PRO, false>(s1, nsmax, sp, dim3(gx, ir.nrows, Z), sint)
+                   : ks_launch_strided<false, PRO, true>(s1, nsmax, sp, dim3(gx, ir.nrows, Z), sint)) return -1; }
+        ProfScope ps(LGPU_KCLASS_EPILOGUE, sint, 8.0 * N * Z * ir.nrows * epi_words, 1);
+        cp.rm = ir;
+        if (pass ? fz_launch_chunk<false, false, RS>(cp, dim3(chunks, ir.nrows, Z), sint)
+                 : fz_launch_chunk<false, true, RS>(cp, dim3(chunks, ir.nrows, Z), sint)) return -1;
+    }
+    if (fp.nrows) {
+        consts(fp);
+        { ProfScope ps(LGPU_KCLASS_FUSED, st, 8.0 * N * Z * fp.nrows, 1);
+          sp.rm = fp; if (ks_launch_strided<true, PRO>(s1, nsmax, sp, dim3(gx, fp.nrows, Z), st)) return -1; }
+        ProfScope ps(LGPU_KCLASS_EPILOGUE, st, 8.0 * N * Z * fp.nrows * epi_words, 1);
+        cp.rm = fp; if (fz_launch_chunk<true, true, RS>(cp, dim3(chunks, fp.nrows, Z), st)) return -1;
+    }
+    join_side(c, st, sint);
+    return 0;
+}
+
 // Fused Evaluator.ModDown (NTT -> NTT, core/rlwe/evaluator_gadget_product.go:39-52 = 2 x ModDownQPtoQNTT,
 // ring/basis_extension.go:235-256) for ncomp x batch QP-stacked accumulators, with an optional addend:
 //     out[c][b] = (accQ[c][b] - NTT(ModUpPtoQ(INTT(accP[c][b])))) * P^-1  (+ D[c][b])
+// rescale = 1: followed by Ring.DivRoundByLastModulusNTT (ring/scaling.go:101-122), out receiving rows 0..levelQ-1. Only row L = levelQ of
+// the ModDown output is formed (a one-row pass into scratch, then its INTT c_L); every other row j takes ONE extension and ONE transform:
+//     out_j = ((acc_j - NTT(E_j)) P^-1 + D_j - NTT(ext_L,j)) q_L^-1  =  (acc_j P^-1 + D_j - NTT(P^-1 E_j + ext_L,j)) q_L^-1   (mod q_j)
+// with E_j the P -> Q extension and ext_L,j = (c_L + floor(q_L/2)) mod q_L - floor(q_L/2) mod q_j the Rescale broadcast term: the K2 prologue
+// PRO_MODUP_BCAST (constants Ctx::muc_PtoQ_pinv) and the RS epilogue. Every step is exact mod q_j, so the output words equal those of the
+// two separate passes.
 int moddown_ntt_fused(const Ctx* c, int levelQ, int levelP, const u64* acc, size_t acc_cs, size_t acc_bs, const u64* D, size_t d_cs, size_t d_bs,
-                      u64* out, size_t o_cs, size_t o_bs, int ncomp, int batch, cudaStream_t st) {
+                      u64* out, size_t o_cs, size_t o_bs, int ncomp, int batch, cudaStream_t st, int rescale) {
+    if (rescale && levelQ < 1) { set_error("cannot Rescale at level 0"); return -1; }
     const int nq = levelQ + 1, np = levelP + 1;
     const size_t N = c->N;
     const int Z = ncomp * batch;
-    const int s1 = c->logN - 12;
-    const size_t bp_words = (size_t)Z * np * N, y_words = bp_words, p1_words = (size_t)Z * nq * N, v_words = ((size_t)Z * N + 7) / 8;
+    // scratch: INTT of the P rows | y | P1 (one row per output row) | v bytes | rescale: ModDown row L and its INTT
+    const size_t bp_words = (size_t)Z * np * N, y_words = bp_words, p1_words = (size_t)Z * (nq - rescale) * N, v_words = ((size_t)Z * N + 7) / 8;
+    const size_t l_words = rescale ? 2 * (size_t)Z * N : 0;
     u64* buf = nullptr;
-    LGPU_CUDA_OK(cudaMallocAsync((void**)&buf, (bp_words + y_words + p1_words + v_words) * sizeof(u64), st));
+    LGPU_CUDA_OK(cudaMallocAsync((void**)&buf, (bp_words + y_words + p1_words + v_words + l_words) * sizeof(u64), st));
     struct Free { u64* p; cudaStream_t s; ~Free() { cudaFreeAsync(p, s); } } guard{buf, st};
     u64* buffP = buf; u64* Y = buffP + bp_words; u64* P1 = Y + y_words;
     unsigned char* V = reinterpret_cast<unsigned char*>(P1 + p1_words);
+    u64* mdL = P1 + p1_words + v_words; u64* cL = mdL + (size_t)Z * N;
     // A: INTT of the P rows
-    RowMap rp;
-    rp.nrows = np;
-    for (int j = 0; j < np; j++) { rp.limb[j] = (unsigned char)(c->nQ + j); rp.drow[j] = (unsigned char)j; }
+    const RowMap rp = q_rows(c->nQ, np);
     for (int cc = 0; cc < ncomp; cc++) {
         CSpan in{acc + (size_t)cc * acc_cs + (size_t)nq * N, N, acc_bs};
         Span o{buffP + (size_t)cc * batch * np * N, N, (size_t)np * N};
@@ -1528,52 +1623,65 @@ int moddown_ntt_fused(const Ctx* c, int levelQ, int levelP, const u64* acc, size
         ks_prepare_kernel<<<dim3((unsigned)((N + 255) / 256), Z), 256, 0, st>>>(pp);
         LGPU_CUDA_OK(cudaGetLastError());
     }
-    // C: basis extension folded into the strided pass
-    RowMap fp, in;
-    split_rows(c, 0, nq, fp, in);
+    // C: basis extension folded into the strided pass, then the chunk-pass epilogue
     KsStridedParams sp;
     memset(&sp, 0, sizeof(sp));
     sp.limbs = c->d_limbs; sp.blob = c->d_blob; sp.Y = Y; sp.y_bs = (size_t)np * N; sp.V = V; sp.v_bs = N;
-    sp.P1 = P1; sp.p1_ds = (size_t)nq * N; sp.p1_bs = (size_t)nq * N;
-    sp.logN = c->logN; sp.nq = nq; sp.k = np; sp.nd = 1; sp.skip_own = 0; sp.single_rule = 0; sp.src_limb0 = c->nQ; sp.split23 = k2_split();
-    sp.dg[0].nS = (unsigned short)np; sp.dg[0].ldc = (unsigned short)m.nS;
-    sp.dg[0].off_c = (unsigned)m.off_qoverqimodp; sp.dg[0].off_vt = (unsigned)m.off_vtimesqmodp; sp.dg[0].off_half_t = (unsigned)m.off_half_t;
-    sp.dg[0].off_cp = (unsigned)m.off_c_plain;
-    {
+    sp.logN = c->logN; sp.k = np; sp.nd = 1; sp.skip_own = 0; sp.single_rule = 0; sp.src_limb0 = c->nQ; sp.split23 = k2_split();
+    auto set_digit = [&](const ModUpSet& s) {
+        sp.dg[0].nS = (unsigned short)np; sp.dg[0].ldc = (unsigned short)s.nS;
+        sp.dg[0].off_c = (unsigned)s.off_qoverqimodp; sp.dg[0].off_vt = (unsigned)s.off_vtimesqmodp; sp.dg[0].off_half_t = (unsigned)s.off_half_t;
+        sp.dg[0].off_cp = (unsigned)s.off_c_plain;
         bool fps = true;
         for (int j = 0; j < np; j++) fps = fps && c->h_limbs[c->nQ + j].fp_ok;
         sp.dg[0].fp_src = fps ? (unsigned short)(1 + k2_fpsum()) : 0;
-    }
+    };
+    set_digit(m);
     FzChunkParams cp;
     memset(&cp, 0, sizeof(cp));
-    cp.limbs = c->d_limbs; cp.P1 = P1; cp.p1_bs = (size_t)nq * N;
-    cp.A = acc; cp.a_cs = acc_cs; cp.a_bs = acc_bs; cp.D = D; cp.d_cs = d_cs; cp.d_bs = d_bs;
-    cp.out = out; cp.o_cs = o_cs; cp.o_bs = o_bs; cp.nb = batch; cp.logN = c->logN;
-    const unsigned gx = (unsigned)(((N >> s1) + 255) / 256);
-    const unsigned chunks = (unsigned)(N >> 12);
-    auto scal = [&](const RowMap& rm) { for (int r = 0; r < rm.nrows; r++) { const int i = rm.drow[r]; cp.s[r] = c->Q[i] - c->mdc_PtoQ[(size_t)levelP * c->nQ + i]; } };
-    cudaStream_t sint = fork_side(c, st, fp.nrows > 0 && in.nrows > 0);
-    RowMap in_c, in_n;
-    split_by_corr(c, in, in_c, in_n);
-    for (int pass = 0; pass < 2; pass++) {
-        const RowMap& ir = pass ? in_n : in_c;
-        if (!ir.nrows) continue;
-        { ProfScope ps(LGPU_KCLASS_FUSED, sint, 8.0 * N * Z * ir.nrows, 1);
-          sp.rm = ir;
-          if (pass ? ks_launch_strided<false, PRO_MODUP, false>(s1, np, sp, dim3(gx, ir.nrows, Z), sint)
-                   : ks_launch_strided<false, PRO_MODUP, true>(s1, np, sp, dim3(gx, ir.nrows, Z), sint)) return -1; }
-        ProfScope ps(LGPU_KCLASS_EPILOGUE, sint, 8.0 * N * Z * ir.nrows * ((D ? 5.0 : 4.0) - 1.0), 1);
-        cp.rm = ir; scal(ir);
-        if (pass ? fz_launch_chunk<false, false>(cp, dim3(chunks, ir.nrows, Z), sint) : fz_launch_chunk<false, true>(cp, dim3(chunks, ir.nrows, Z), sint)) return -1;
+    cp.limbs = c->d_limbs; cp.nb = batch; cp.logN = c->logN;
+    const u64* mdc = &c->mdc_PtoQ[(size_t)levelP * c->nQ];
+    auto md_consts = [&](const RowMap& rm) { for (int r = 0; r < rm.nrows; r++) { const int i = rm.limb[r]; cp.s[r] = c->Q[i] - mdc[i]; } };
+    const double md_words = D ? 4.0 : 3.0;      // P1 + accumulator (+ D) read, out written
+    if (!rescale) {
+        sp.P1 = P1; sp.p1_ds = sp.p1_bs = (size_t)nq * N; sp.nq = nq;
+        cp.P1 = P1; cp.p1_bs = (size_t)nq * N;
+        cp.A = acc; cp.a_cs = acc_cs; cp.a_bs = acc_bs; cp.D = D; cp.d_cs = d_cs; cp.d_bs = d_bs;
+        cp.out = out; cp.o_cs = o_cs; cp.o_bs = o_bs;
+        return fz_tail<PRO_MODUP, false>(c, q_rows(0, nq), np, sp, cp, Z, md_words, md_consts, st);
     }
-    if (fp.nrows) {
-        { ProfScope ps(LGPU_KCLASS_FUSED, st, 8.0 * N * Z * fp.nrows, 1);
-          sp.rm = fp; if (ks_launch_strided<true>(s1, np, sp, dim3(gx, fp.nrows, Z), st)) return -1; }
-        ProfScope ps(LGPU_KCLASS_EPILOGUE, st, 8.0 * N * Z * fp.nrows * ((D ? 5.0 : 4.0) - 1.0), 1);
-        cp.rm = fp; scal(fp); if (fz_launch_chunk<true>(cp, dim3(chunks, fp.nrows, Z), st)) return -1;
-    }
-    join_side(c, st, sint);
-    return 0;
+    const int L = levelQ;
+    // C1: ModDown of row L alone into mdL [Z][N] (launch row 0: the row offsets are folded into the pointers), then c_L = INTT(mdL)
+    RowMap rl;
+    rl.nrows = 1; rl.limb[0] = (unsigned char)L; rl.drow[0] = 0;
+    sp.P1 = P1; sp.p1_ds = sp.p1_bs = N; sp.nq = 1;
+    cp.P1 = P1; cp.p1_bs = N;
+    cp.A = acc + (size_t)L * N; cp.a_cs = acc_cs; cp.a_bs = acc_bs;
+    cp.D = D ? D + (size_t)L * N : nullptr; cp.d_cs = d_cs; cp.d_bs = d_bs;
+    cp.out = mdL; cp.o_cs = (size_t)batch * N; cp.o_bs = N;
+    if (fz_tail<PRO_MODUP, false>(c, rl, np, sp, cp, Z, md_words, md_consts, st)) return -1;
+    if (launch_intt(c, rl, CSpan{mdL, N, N}, Span{cL, N, N}, Z, NTT_CANONICAL, st)) return -1;
+    // C2: rows 0..L-1, one extension (P^-1 E_j + ext_L,j) and one transform each, straight into out
+    const u64 qL = c->Q[L];
+    const u64 pHalf = (qL - 1) >> 1;
+    set_digit(c->muc_PtoQ_pinv[levelP]);
+    sp.P1 = P1; sp.p1_ds = sp.p1_bs = (size_t)L * N; sp.nq = L;
+    sp.bc = cL; sp.bc_bs = N; sp.bc_add = pHalf; sp.bc_q = qL;
+    cp.P1 = P1; cp.p1_bs = (size_t)L * N;
+    cp.A = acc; cp.D = D;
+    cp.out = out; cp.o_cs = o_cs; cp.o_bs = o_bs;
+    const u64* resc = &c->rescaleQ[(size_t)(L - 1) * c->nQ];
+    auto rs_consts = [&](const RowMap& rm) {
+        for (int r = 0; r < rm.nrows; r++) {
+            const int i = rm.limb[r];
+            const u64 qi = c->Q[i];
+            sp.s0[r] = qi - (pHalf % qi);
+            cp.s[r] = resc[i];
+            // MForm(P^-1 q_L^-1) = MForm(P^-1) * (-RescaleConstant) * 2^-64: both are Montgomery forms
+            cp.s2[r] = h_mulmod(h_mulmod(mdc[i], (qi - resc[i]) % qi, qi), h_invmod(h_mform(1, qi), qi), qi);
+        }
+    };
+    return fz_tail<PRO_MODUP_BCAST, true>(c, q_rows(0, L), np, sp, cp, Z, md_words, rs_consts, st);
 }
 
 // Fused Ring.DivRoundByLastModulusNTT (ring/scaling.go:101-122) for ncomp x batch polynomials at level `level`:
@@ -1582,7 +1690,6 @@ int div_round_last_ntt_fused(const Ctx* c, int level, const u64* X, size_t x_cs,
                              int ncomp, int batch, cudaStream_t st) {
     const size_t N = c->N;
     const int Z = ncomp * batch;
-    const int s1 = c->logN - 12;
     u64* buf = nullptr;
     LGPU_CUDA_OK(cudaMallocAsync((void**)&buf, ((size_t)Z * N + (size_t)Z * level * N) * sizeof(u64), st));
     struct Free { u64* p; cudaStream_t s; ~Free() { cudaFreeAsync(p, s); } } guard{buf, st};
@@ -1596,8 +1703,6 @@ int div_round_last_ntt_fused(const Ctx* c, int level, const u64* X, size_t x_cs,
     }
     const u64 qL = c->Q[level];
     const u64 pHalf = (qL - 1) >> 1;
-    RowMap fp, in;
-    split_rows(c, 0, level, fp, in);
     KsStridedParams sp;
     memset(&sp, 0, sizeof(sp));
     sp.limbs = c->d_limbs; sp.blob = c->d_blob; sp.P1 = P1; sp.p1_ds = (size_t)level * N; sp.p1_bs = (size_t)level * N;
@@ -1608,32 +1713,14 @@ int div_round_last_ntt_fused(const Ctx* c, int level, const u64* X, size_t x_cs,
     cp.limbs = c->d_limbs; cp.P1 = P1; cp.p1_bs = (size_t)level * N;
     cp.A = X; cp.a_cs = x_cs; cp.a_bs = x_bs; cp.D = nullptr;
     cp.out = out; cp.o_cs = o_cs; cp.o_bs = o_bs; cp.nb = batch; cp.logN = c->logN;
-    const unsigned gx = (unsigned)(((N >> s1) + 255) / 256);
-    const unsigned chunks = (unsigned)(N >> 12);
-    auto s0 = [&](const RowMap& rm) { for (int k = 0; k < rm.nrows; k++) { const u64 qi = c->Q[rm.drow[k]]; sp.s0[k] = qi - (pHalf % qi); } };
-    auto scal = [&](const RowMap& rm) { for (int k = 0; k < rm.nrows; k++) cp.s[k] = c->rescaleQ[(size_t)(level - 1) * c->nQ + rm.drow[k]]; };
-    cudaStream_t sint = fork_side(c, st, fp.nrows > 0 && in.nrows > 0);
-    RowMap in_c, in_n;
-    split_by_corr(c, in, in_c, in_n);
-    for (int pass = 0; pass < 2; pass++) {
-        const RowMap& ir = pass ? in_n : in_c;
-        if (!ir.nrows) continue;
-        { ProfScope ps(LGPU_KCLASS_FUSED, sint, 8.0 * N * Z * ir.nrows, 1);
-          sp.rm = ir; s0(ir);
-          if (pass ? ks_launch_strided<false, PRO_BCAST, false>(s1, 1, sp, dim3(gx, ir.nrows, Z), sint)
-                   : ks_launch_strided<false, PRO_BCAST, true>(s1, 1, sp, dim3(gx, ir.nrows, Z), sint)) return -1; }
-        ProfScope ps(LGPU_KCLASS_EPILOGUE, sint, 8.0 * N * Z * ir.nrows * (4.0 - 1.0), 1);
-        cp.rm = ir; scal(ir);
-        if (pass ? fz_launch_chunk<false, false>(cp, dim3(chunks, ir.nrows, Z), sint) : fz_launch_chunk<false, true>(cp, dim3(chunks, ir.nrows, Z), sint)) return -1;
-    }
-    if (fp.nrows) {
-        { ProfScope ps(LGPU_KCLASS_FUSED, st, 8.0 * N * Z * fp.nrows, 1);
-          sp.rm = fp; s0(fp); if (ks_launch_strided<true, PRO_BCAST>(s1, 1, sp, dim3(gx, fp.nrows, Z), st)) return -1; }
-        ProfScope ps(LGPU_KCLASS_EPILOGUE, st, 8.0 * N * Z * fp.nrows * (4.0 - 1.0), 1);
-        cp.rm = fp; scal(fp); if (fz_launch_chunk<true>(cp, dim3(chunks, fp.nrows, Z), st)) return -1;
-    }
-    join_side(c, st, sint);
-    return 0;
+    auto consts = [&](const RowMap& rm) {
+        for (int k = 0; k < rm.nrows; k++) {
+            const u64 qi = c->Q[rm.drow[k]];
+            sp.s0[k] = qi - (pHalf % qi);
+            cp.s[k] = c->rescaleQ[(size_t)(level - 1) * c->nQ + rm.drow[k]];
+        }
+    };
+    return fz_tail<PRO_BCAST, false>(c, q_rows(0, level), 1, sp, cp, Z, 3.0, consts, st);
 }
 
 }  // namespace lgpu

@@ -194,6 +194,23 @@ static ModUpSet gen_modup(std::vector<u64>& blob, const u64* S, int nS, const u6
     return m;
 }
 
+// A copy of the target-side constants of `m` multiplied by s[j] mod T[j], appended to the blob. The basis extension is linear in
+// them (sum_i y_i (S/s_i mod t_j) - v S - S/2), so the copy evaluates s[j] times the extension.
+static ModUpSet scale_modup_targets(std::vector<u64>& blob, const ModUpSet& m, const u64* s, const u64* T) {
+    ModUpSet r = m;
+    auto scaled = [&](size_t off, int per_target) {
+        const size_t out = blob.size();
+        for (int j = 0; j < m.nT; j++)
+            for (int i = 0; i < per_target; i++) blob.push_back(h_mulmod(blob[off + (size_t)j * per_target + i], s[j], T[j]));
+        return out;
+    };
+    r.off_qoverqimodp = scaled(m.off_qoverqimodp, m.nS);
+    r.off_vtimesqmodp = scaled(m.off_vtimesqmodp, m.nS + 1);
+    r.off_half_t = scaled(m.off_half_t, 1);
+    r.off_c_plain = scaled(m.off_c_plain, m.nS);
+    return r;
+}
+
 int ensure_scratch(Ctx* c, size_t words) {
     if (words <= c->scratch_words) return 0;
     if (c->d_scratch) {
@@ -305,6 +322,16 @@ int build_context(Ctx* c, int device, int logN, int ring_type, const u64* q, int
         for (int i = 0; i < nq; i++) c->muc_QtoP[i] = gen_modup(c->h_blob, q, i + 1, p, np);
         c->muc_PtoQ.resize(np);
         for (int i = 0; i < np; i++) c->muc_PtoQ[i] = gen_modup(c->h_blob, p, i + 1, q, nq);
+        c->muc_PtoQ_pinv.resize(np);
+        for (int i = 0; i < np; i++) {
+            std::vector<u64> pinv(nq);
+            for (int j = 0; j < nq; j++) {
+                u64 pr = 1;
+                for (int u = 0; u <= i; u++) pr = h_mulmod(pr, p[u] % q[j], q[j]);
+                pinv[j] = h_invmod(pr, q[j]);
+            }
+            c->muc_PtoQ_pinv[i] = scale_modup_targets(c->h_blob, c->muc_PtoQ[i], pinv.data(), q);
+        }
         // genmodDownConstants: [j][i] = MForm((p_0..p_j)^-1 mod q_i)
         c->mdc_PtoQ.assign((size_t)np * nq, 0);
         for (int i = 0; i < nq; i++) {
